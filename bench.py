@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          # our arm (CUDA, through the C ABI)
   python bench.py --impl reference --gpus N ...          # the CPU arm on the box's host cores
+  python bench.py ... --dump-outputs DIR                  # also write what the last timed step computed, DIR/<name>.npy
 
 One "step" = one pass of State::ApplyAction over one batch of 1,048,576 connect_four states (SoA, 16 B per
 state) with one legal action per state.  The (state, action) stream is synthetic: every lane is advanced
@@ -340,6 +341,7 @@ def run_gpu(args):
     ms_apply_total = time_graphs(lambda i: works[i].apply_actions(acts[i]), n_streams=2)
     for w_ in works:
         w_.check_errors()
+    outputs = step_outputs(torch, works[W + (K - 1) % C], dev) if args.dump_outputs and rank == 0 else None
     ms_apply_s1 = time_graphs(lambda i: works[i].apply_actions(acts[i]), reps=2, n_streams=1)
     ms_apply_s4 = time_graphs(lambda i: works[i].apply_actions(acts[i]), reps=2, n_streams=4)
     for w_ in works:
@@ -598,10 +600,37 @@ def run_gpu(args):
                    "launches_total_incl_setup": total_launches, "loops": loops, "cpu_reference_loops": cpu_loops()},
         "clocks": sampler.summary() if sampler else None,
     }
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_OBS_LANES = 4096
+
+
+def step_outputs(torch, batch, dev):
+    """What a caller of the timed ApplyAction step reads back from the batch it advanced: player to move, terminal flag,
+    returns and legal-action mask of every lane, and the observation tensor of a fixed, seeded sample of lanes (all of it
+    would be 504 MiB)."""
+    cur, term, rets = batch.status()
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(0x0B5)
+    lanes = torch.randperm(batch.n, device=dev, generator=gen)[:DUMP_OBS_LANES].sort().values
+    obs = batch.observation_tensor(player=0)[lanes]
+    mask = batch.legal_actions_mask_words().to(torch.int64) & 0xFFFFFFFF
+    return {"current_player": cur.to(torch.float32), "terminal": term.to(torch.float32), "returns": rets.to(torch.float32),
+            "legal_mask_words": mask.to(torch.float64), "observation_lanes": lanes.to(torch.float64),
+            "observation_sample": obs.to(torch.float32)}
+
+
+def dump_outputs(directory, outputs):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
 
 
 def main():
@@ -613,7 +642,10 @@ def main():
     ap.add_argument("--deep-trees", type=int, default=8192, help="trees per GPU of the deep MCTS line")
     ap.add_argument("--deep-sims", type=int, default=10000, help="simulations per tree of the deep MCTS line")
     ap.add_argument("--cfr-iters", type=int, default=100000, help="CFRSolver iterations (BASELINE configs[3]: 100k)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)

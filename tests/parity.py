@@ -8,6 +8,7 @@ import torch
 
 import open_spiel_b200 as b2
 from oracle_lib import OracleGame
+from reference_golden import Digest
 
 
 def mask_words_to_lists(words, width):
@@ -20,17 +21,21 @@ def mask_words_to_lists(words, width):
 
 def lockstep(game_string, n_lanes=512, seed=0, check_obs_every=3, max_plies=None, check_info_state=False,
              checker=OracleGame):
-    """Play n_lanes random games in lock-step on device and on the checker (the oracle restatement, or — passing
-    ref_lib.RefGame — the unmodified reference build); assert equality of everything after every move."""
+    """Play n_lanes random games in lock-step on device and on the checker (the oracle restatement); assert equality of
+    everything after every move.  checker=None: no checker; returns (steps, digest of everything a checker would have been
+    compared with), to hold against checker_digest() of a checker that is not at hand (the unmodified reference)."""
     rng = np.random.RandomState(seed)
     game = b2.load_game(game_string)
-    ogame = checker(game_string)
-    assert game.num_distinct_actions() == ogame.num_distinct_actions
-    assert game.max_game_length() == ogame.max_game_length
-    assert game.num_players() == ogame.num_players
-    assert game.observation_tensor_size() == ogame.observation_tensor_size
+    record = Digest(_header(game.num_distinct_actions(), game.max_game_length(), game.num_players(),
+                            game.observation_tensor_size())) if checker is None else None
+    if checker is not None:
+        ogame = checker(game_string)
+        assert game.num_distinct_actions() == ogame.num_distinct_actions
+        assert game.max_game_length() == ogame.max_game_length
+        assert game.num_players() == ogame.num_players
+        assert game.observation_tensor_size() == ogame.observation_tensor_size
     batch = game.new_batch(n_lanes)
-    ostates = [ogame.new_initial_state() for _ in range(n_lanes)]
+    ostates = [ogame.new_initial_state() for _ in range(n_lanes)] if checker is not None else [None] * n_lanes
     width = max(game.num_distinct_actions(), game.max_chance_outcomes())
     P = game.num_players()
     dev = batch._dev
@@ -50,6 +55,14 @@ def lockstep(game_string, n_lanes=512, seed=0, check_obs_every=3, max_plies=None
         actions = np.full(n_lanes, -1, dtype=np.int32)
         alive = 0
         for i, st in enumerate(ostates):
+            if st is None:
+                _record(record, cur[i], term[i], legal[i], rets[i].tolist(), obs and [o[i] for o in obs],
+                        obs and check_info_state and [t[i] for t in ist])
+                assert counts[i] == len(legal[i]) and acts_l[i, :len(legal[i])].tolist() == legal[i]
+                if not term[i]:
+                    actions[i] = legal[i][rng.randint(len(legal[i]))]
+                    alive += 1
+                continue
             assert int(cur[i]) == st.current_player(), (game_string, "current_player", i, ply)
             assert bool(term[i]) == st.is_terminal(), (game_string, "is_terminal", i, ply)
             ola = st.legal_actions()
@@ -86,4 +99,37 @@ def lockstep(game_string, n_lanes=512, seed=0, check_obs_every=3, max_plies=None
         assert cnt == 0, (game_string, "unexpected rejected lanes", cnt, first)
         ply += 1
         assert ply <= limit, "game did not end"
-    return total_steps
+    return total_steps if record is None else (total_steps, record.hexdigest())
+
+
+def _header(num_distinct_actions, max_game_length, num_players, observation_tensor_size):
+    return [num_distinct_actions, max_game_length, num_players, observation_tensor_size]
+
+
+def _record(d, cur, term, legal, rets, obs, ist):
+    d.add(int(cur), bool(term), legal, [float(x).hex() for x in rets], obs or None, ist or None)
+
+
+def checker_digest(game_string, checker, n_lanes=512, seed=0, check_obs_every=3, max_plies=None, check_info_state=False):
+    """The checker's side of lockstep(checker=None): its states played the same way, observed the same way."""
+    rng = np.random.RandomState(seed)
+    g = checker(game_string)
+    d = Digest(_header(g.num_distinct_actions, g.max_game_length, g.num_players, g.observation_tensor_size))
+    states = [g.new_initial_state() for _ in range(n_lanes)]
+    P = g.num_players
+    ply = 0
+    while True:
+        check = check_obs_every and ply % check_obs_every == 0
+        actions = []
+        for st in states:
+            la = st.legal_actions()
+            _record(d, st.current_player(), st.is_terminal(), la, st.returns(),
+                    check and [st.observation_tensor(p) for p in range(P)],
+                    check and check_info_state and [st.information_state_tensor(p) for p in range(P)])
+            actions.append(None if st.is_terminal() else la[rng.randint(len(la))])
+        if all(a is None for a in actions):
+            return d.hexdigest()
+        for st, a in zip(states, actions):
+            if a is not None:
+                st.apply_action(a)
+        ply += 1

@@ -1,8 +1,9 @@
 """Parity of the BENCHED workload itself (SURVEY §8d config 2: "first 1M lanes replayed through the oracle"): the exact
 1,048,576-lane U{0..20}-ply connect_four batch bench.py times (same builder, same seed) is replayed lane by lane on the
-UNMODIFIED reference (oracle/_ref), and every output of the benched step — legal mask before, terminal, current player,
-returns, next legal mask and the full observation tensor after — must match on every lane.  Both host entry points
-(float and compact) are checked on the same batch."""
+UNMODIFIED reference, and every output of the benched step — legal mask before, terminal, current player, returns, next
+legal mask and the full observation tensor after — must match on every lane.  The reference's outputs are stored as
+digests (tests/reference_golden.py), with digests of the batch they were computed on.  Both host entry points (float and
+compact) are checked on the same batch."""
 import os
 import sys
 
@@ -10,24 +11,42 @@ import numpy as np
 import pytest
 import torch
 
-import ref_lib
+from reference_golden import digest, expected
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not built")
-def test_benched_connect_four_batch_equals_reference_on_every_lane():
+def benched_batch():
     import bench
     import open_spiel_b200 as b2
+    game = b2.Game("connect_four", device=0)
+    _, snap, actions, hist = bench.build_workload(torch, game, bench.N_STATES, torch.device("cuda", 0), seed=0x5EED,
+                                                  with_history=True)
+    return game, snap, actions, hist
+
+
+def reference_golden():
+    """Needs a CUDA device: the batch is built there, as bench.py builds it, and replayed on the reference."""
+    import ref_lib
+    _, _, actions, hist = benched_batch()
+    hist, actions = hist.cpu().numpy(), actions.cpu().numpy()
+    ref = ref_lib.replay_batch("connect_four", hist, actions, mask_words=1)
+    assert ref["failed_lanes"] == 0
+    out = {"batch": digest(hist, actions), "terminal_count": int(ref["terminal"].sum())}
+    out.update({k: digest(ref[k]) for k in ("mask_before", "terminal", "cur_player", "returns", "mask_after", "obs_bits")})
+    return {"gpu_bench_workload/connect_four": out}
+
+
+def test_benched_connect_four_batch_equals_reference_on_every_lane():
+    import bench
+    ref = expected("gpu_bench_workload/connect_four")
     n = bench.N_STATES
     dev = torch.device("cuda", 0)
-    game = b2.Game("connect_four", device=0)
-    _, snap, actions, hist = bench.build_workload(torch, game, n, dev, seed=0x5EED, with_history=True)
+    game, snap, actions, hist = benched_batch()
     assert hist.shape == (n, bench.MAX_PREFIX)
-    ref = ref_lib.replay_batch("connect_four", hist.cpu().numpy(), actions.cpu().numpy(), mask_words=1)
-    assert ref["failed_lanes"] == 0
+    assert digest(hist.cpu().numpy(), actions.cpu().numpy()) == ref["batch"]      # the batch the reference replayed
     # the device step on the benched batch
     work = game.new_batch(n)
     work.copy_from(snap)
@@ -39,19 +58,21 @@ def test_benched_connect_four_batch_equals_reference_on_every_lane():
     work.check_errors()
     cur, term2, rets2 = work.status()
     obs = work.observation_tensor(player=0)                       # [n, 126] float32
-    assert np.array_equal(mask_before, ref["mask_before"])
-    assert np.array_equal(term.cpu().numpy(), ref["terminal"])
-    assert np.array_equal(term2.cpu().numpy(), ref["terminal"])
-    assert np.array_equal(cur.cpu().numpy(), ref["cur_player"])
-    assert np.array_equal(rets.cpu().numpy(), ref["returns"]) and np.array_equal(rets2.cpu().numpy(), ref["returns"])
-    assert np.array_equal(mask.cpu().numpy().astype(np.uint32), ref["mask_after"])
+    assert digest(mask_before) == ref["mask_before"]
+    terminal = term.cpu().numpy()
+    assert digest(terminal) == ref["terminal"] and np.array_equal(term2.cpu().numpy(), terminal)
+    assert digest(cur.cpu().numpy()) == ref["cur_player"]
+    returns = rets.cpu().numpy()
+    assert digest(returns) == ref["returns"] and np.array_equal(rets2.cpu().numpy(), returns)
+    mask_after = mask.cpu().numpy().astype(np.uint32)
+    assert digest(mask_after) == ref["mask_after"]
     F = obs.shape[1]
     pad = torch.zeros((n, (-F) % 32), dtype=obs.dtype, device=dev)
     bits = (torch.cat([obs, pad], dim=1) != 0).reshape(n, -1, 32).to(torch.int64)
     words = (bits << torch.arange(32, device=dev, dtype=torch.int64)).sum(dim=2).cpu().numpy().astype(np.uint32)
-    assert np.array_equal(words, ref["obs_bits"])
-    assert int(ref["terminal"].sum()) > 0 and int((ref["terminal"] == 0).sum()) > n // 2      # the step does end some games
-    # the two host entry points on the same batch
+    assert digest(words) == ref["obs_bits"]
+    assert ref["terminal_count"] == int(terminal.sum()) > 0 and int((terminal == 0).sum()) > n // 2   # the step does end some games
+    # the two host entry points on the same batch, against the outputs just matched with the reference
     work.copy_from(snap)
     act_h = actions.cpu().pin_memory()
     mask_h = torch.empty((n, 1), dtype=torch.int32).pin_memory()
@@ -59,17 +80,17 @@ def test_benched_connect_four_batch_equals_reference_on_every_lane():
     rets_h = torch.empty((n, 2), dtype=torch.float32).pin_memory()
     torch.cuda.synchronize()
     work.step_host(act_h, mask_h, term_h, rets_h)
-    assert np.array_equal(term_h.numpy(), ref["terminal"]) and np.array_equal(rets_h.numpy(), ref["returns"])
-    assert np.array_equal(mask_h.numpy().astype(np.uint32), ref["mask_after"])
+    assert np.array_equal(term_h.numpy(), terminal) and np.array_equal(rets_h.numpy(), returns)
+    assert np.array_equal(mask_h.numpy().astype(np.uint32), mask_after)
     work.copy_from(snap)
     torch.cuda.synchronize()
     status_h = torch.empty((n,), dtype=torch.uint8).pin_memory()
     work.step_host_compact(actions.to(torch.uint8).cpu().pin_memory(), status_h)
     st = status_h.numpy()
-    t = ref["terminal"].astype(bool)
-    assert np.array_equal(st >> 7, ref["terminal"])
-    assert np.array_equal(st[~t] & 0x7F, ref["mask_after"][~t, 0].astype(np.uint8))
-    outcome = np.where(ref["returns"][:, 0] > 0, 1, np.where(ref["returns"][:, 0] < 0, 2, 0)).astype(np.uint8)
+    t = terminal.astype(bool)
+    assert np.array_equal(st >> 7, terminal)
+    assert np.array_equal(st[~t] & 0x7F, mask_after[~t, 0].astype(np.uint8))
+    outcome = np.where(returns[:, 0] > 0, 1, np.where(returns[:, 0] < 0, 2, 0)).astype(np.uint8)
     assert np.array_equal(st[t] & 3, outcome[t])
     work.check_errors()
 

@@ -200,10 +200,8 @@ def test_device_mcts_matches_reference_mctsbot_in_distribution():
     """The reference's RNG streams (std::shuffle, absl::Uniform) cannot be reproduced (SURVEY §8c), so against the
     UNMODIFIED MCTSBot the comparison is statistical: over many independent searches of the same connect_four
     position, the mean share of simulations each root action receives must agree (uct_c = 2, 400 simulations, no
-    solver), and so must the mean root value."""
-    import ref_lib
-    if not ref_lib.available():
-        pytest.skip("oracle/_ref not shipped")
+    solver), and so must the mean root value.  The reference's means are stored (tests/reference_golden.py)."""
+    from reference_golden import expected
     gs, prefix = "connect_four", [3, 3, 2]
     sims, trees = 400, 512
     game = b2.load_game(gs)
@@ -214,19 +212,27 @@ def test_device_mcts_matches_reference_mctsbot_in_distribution():
     v = out["visits"].double()
     dev_share = (v / v.sum(dim=1, keepdim=True)).mean(dim=0).cpu().numpy()
     dev_value = float((out["total_reward"].sum(dim=1) / v.sum(dim=1)).mean())
-    rg = ref_lib.RefGame(gs)
+    ref = expected("gpu_mcts/connect_four")
+    share, value = np.array(ref["share"]), ref["value"]
+    # standard error of a mean share over a few hundred searches is ~0.005; allow 0.03
+    assert np.abs(dev_share - share).max() < 0.03, (dev_share, share)
+    assert abs(dev_value - value) < 0.05, (dev_value, value)
+
+
+def reference_golden():
+    """The unmodified MCTSBot's mean root shares and value over 256 searches (seeds 1..256) of the position above."""
+    import ref_lib
+    rg = ref_lib.RefGame("connect_four")
     st = rg.new_initial_state()
-    for a in prefix:
+    for a in [3, 3, 2]:
         st.apply_action(a)
     n_ref = 256
     share = np.zeros(7)
     value = 0.0
     for seed in range(n_ref):
-        r = ref_lib.ref_mcts(rg, st, 2.0, sims, 1, False, seed + 1)
+        r = ref_lib.ref_mcts(rg, st, 2.0, 400, 1, False, seed + 1)
         tot = sum(vv for _, vv, _ in r["children"])
         for a, vv, _ in r["children"]:
             share[a] += vv / tot / n_ref
         value += sum(rw for _, _, rw in r["children"]) / tot / n_ref
-    # standard error of a mean share over a few hundred searches is ~0.005; allow 0.03
-    assert np.abs(dev_share - share).max() < 0.03, (dev_share, share)
-    assert abs(dev_value - value) < 0.05, (dev_value, value)
+    return {"gpu_mcts/connect_four": {"share": share.tolist(), "value": value}}

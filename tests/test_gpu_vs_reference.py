@@ -1,13 +1,13 @@
-"""GPU parity directly against the UNMODIFIED reference (oracle/_ref/libspiel_ref_c.so, shipped with the snapshot):
-the same lock-step harness as test_gpu_parity_games.py with the real open_spiel::State objects as the checker.
+"""GPU parity directly against the UNMODIFIED reference: the same lock-step harness as test_gpu_parity_games.py with the
+real open_spiel::State objects as the checker, their side stored as a digest (tests/reference_golden.py).
 Also: size-independent properties at full batch sizes, and ragged / empty batches."""
 import numpy as np
 import pytest
 import torch
 
 import open_spiel_b200 as b2
-import ref_lib
-from parity import lockstep
+from parity import checker_digest, lockstep
+from reference_golden import expected
 
 pytestmark = pytest.mark.gpu
 
@@ -16,11 +16,16 @@ GAMES = [("tic_tac_toe", 128), ("connect_four", 128), ("breakthrough", 64), ("he
          ("mnk", 16), ("mnk(m=5,n=4,k=3)", 64), ("othello", 64), ("y(board_size=9)", 64), ("havannah(board_size=4,swap=True)", 64), ("havannah", 16)]
 
 
-@pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not shipped")
+def reference_golden():
+    import ref_lib
+    return {"gpu_vs_reference/" + gs: checker_digest(gs, ref_lib.RefGame, n_lanes=lanes, seed=99,
+                                                     check_info_state=gs in ("kuhn_poker", "leduc_poker")) for gs, lanes in GAMES}
+
+
 @pytest.mark.parametrize("gs,lanes", GAMES, ids=[g for g, _ in GAMES])
 def test_device_equals_unmodified_reference(gs, lanes):
-    steps = lockstep(gs, n_lanes=lanes, seed=99, checker=ref_lib.RefGame,
-                     check_info_state=gs in ("kuhn_poker", "leduc_poker"))
+    steps, digest = lockstep(gs, n_lanes=lanes, seed=99, checker=None, check_info_state=gs in ("kuhn_poker", "leduc_poker"))
+    assert digest == expected("gpu_vs_reference/" + gs)
     assert steps > lanes
 
 

@@ -2,37 +2,51 @@
 ExternalSamplingMCCFRSolver (algorithms/external_sampling_mccfr.cc, built by oracle/ref_build.mk).  Fed the reference's own
 random stream (std::mt19937 + std::uniform_real_distribution, both libstdc++), one traversal per update, the restatement
 must reproduce the reference's tables BIT FOR BIT — same information states visited, same cumulative regrets, same
-cumulative policy."""
+cumulative policy.  The reference's tables are stored as digests (tests/reference_golden.py)."""
 import pytest
 
 from oracle_lib import OracleGame, OracleMCCFR
-import ref_lib
+from reference_golden import digest, expected
 
-pytestmark = pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not built")
+CASES = [("kuhn_poker", 0, [1, 9, 90, 900]), ("kuhn_poker", 12345, [50, 500]), ("leduc_poker", 0, [1, 20, 400]), ("leduc_poker", 7, [1000])]
 
 
-@pytest.mark.parametrize("name,seed,steps", [("kuhn_poker", 0, [1, 9, 90, 900]), ("kuhn_poker", 12345, [50, 500]),
-                                             ("leduc_poker", 0, [1, 20, 400]), ("leduc_poker", 7, [1000])])
-def test_oracle_mccfr_equals_reference_bitwise(name, seed, steps):
-    ref = ref_lib.RefMCCFR(ref_lib.RefGame(name), seed)
-    mine = OracleMCCFR(OracleGame(name), seed=seed, rng_mode=0, traversals_per_update=1)
+def table_digest(t):
+    return digest({k: [v["legal"], v["regrets"], v["cum_policy"]] for k, v in t.items()})
+
+
+def checkpoints(solver, steps):
+    out = []
     for k in steps:
-        ref.iterate(k)
-        mine.iterate(k)
-        rt, mt = ref.table(), mine.table()
-        assert set(rt) == set(mt)
-        for key, v in rt.items():
-            assert v["legal"] == mt[key]["legal"]
-            assert v["regrets"] == mt[key]["regrets"], (key, v["regrets"], mt[key]["regrets"])
-            assert v["cum_policy"] == mt[key]["cum_policy"], key
+        solver.iterate(k)
+        out.append(table_digest(solver.table()))
+    return out
+
+
+def reference_golden():
+    import ref_lib
+    out = {"mccfr/%s-%d" % (name, seed): checkpoints(ref_lib.RefMCCFR(ref_lib.RefGame(name), seed), steps)
+           for name, seed, steps in CASES}
+    ref = ref_lib.RefMCCFR(ref_lib.RefGame("kuhn_poker"), 39823987)
+    ref.iterate(1000)
+    out["mccfr/known_answer/kuhn_poker"] = {"nash_conv": ref.nash_conv(), "table": table_digest(ref.table())}
+    return out
+
+
+@pytest.mark.parametrize("name,seed,steps", CASES)
+def test_oracle_mccfr_equals_reference_bitwise(name, seed, steps):
+    mine = OracleMCCFR(OracleGame(name), seed=seed, rng_mode=0, traversals_per_update=1)
+    assert checkpoints(mine, steps) == expected("mccfr/%s-%d" % (name, seed))
 
 
 def test_reference_known_answer_kuhn_nash_conv():
     """external_sampling_mccfr_test.cc: 1000 iterations on kuhn_poker reach NashConv < 0.05 (loose bound of the reference
     test); the restatement with the same stream has the same tables, so the same NashConv."""
-    ref = ref_lib.RefMCCFR(ref_lib.RefGame("kuhn_poker"), 39823987)
-    ref.iterate(1000)
-    assert ref.nash_conv() < 0.1
+    want = expected("mccfr/known_answer/kuhn_poker")
+    assert want["nash_conv"] < 0.1
+    mine = OracleMCCFR(OracleGame("kuhn_poker"), seed=39823987, rng_mode=0, traversals_per_update=1)
+    mine.iterate(1000)
+    assert table_digest(mine.table()) == want["table"]
 
 
 def test_position_keyed_stream_batches_are_order_independent():

@@ -3,15 +3,14 @@ oracle/ref_build.mk).  Fed the reference's own random streams — std::mt19937(s
 children) and for the RandomRolloutEvaluator (absl::Uniform over the legal actions) — the restatement must reproduce the
 search BIT FOR BIT: the root's children in the same (shuffled) order, their visit counts, their total rewards as exact
 doubles, and BestChild.  The device kernel is then compared with the same oracle code on the Philox stream
-(tests/test_gpu_mcts.py): the two modes differ only in where the random integers come from."""
+(tests/test_gpu_mcts.py): the two modes differ only in where the random integers come from.  The reference's searches are
+stored (tests/reference_golden.py)."""
 import random
 
 import pytest
 
 from oracle_lib import OracleGame, oracle_mcts
-import ref_lib
-
-pytestmark = pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not built")
+from reference_golden import expected
 
 CASES = [
     # game, prefix plies, simulations, n_rollouts, solve, seed
@@ -34,21 +33,39 @@ CASES = [
 ]
 
 
-@pytest.mark.parametrize("gs,prefix,sims,nroll,solve,seed", CASES, ids=["%s-%d" % (c[0], c[2]) for c in CASES])
-def test_oracle_mcts_equals_reference_mctsbot_bitwise(gs, prefix, sims, nroll, solve, seed):
+GC_CASES = [("connect_four", 12000, 3), ("hex(board_size=4)", 9000, 5)]
+
+
+def start(game, gs, prefix, seed):
     rng = random.Random(seed)
-    rg, og = ref_lib.RefGame(gs), OracleGame(gs)
-    rs, os_ = rg.new_initial_state(), og.new_initial_state()
+    s = game.new_initial_state()
     for _ in range(prefix):
-        a = rng.choice(rs.legal_actions())
-        nxt = rs.clone()
+        a = rng.choice(s.legal_actions())
+        nxt = s.clone()
         nxt.apply_action(a)
         if nxt.is_terminal():
             break
-        rs.apply_action(a)
-        os_.apply_action(a)
-    ref = ref_lib.ref_mcts(rg, rs, 2.0, sims, nroll, solve, seed)
-    mine = oracle_mcts(os_, 2.0, sims, nroll, solve, seed, reference_rng=True)
+        s.apply_action(a)
+    return s
+
+
+def reference_golden():
+    import ref_lib
+    out = {}
+    for gs, prefix, sims, nroll, solve, seed in CASES:
+        rg = ref_lib.RefGame(gs)
+        out["mcts/%s-%d" % (gs, sims)] = ref_lib.ref_mcts(rg, start(rg, gs, prefix, seed), 2.0, sims, nroll, solve, seed)
+    for gs, sims, seed in GC_CASES:
+        rg = ref_lib.RefGame(gs)
+        r = ref_lib.ref_mcts(rg, rg.new_initial_state(), 2.0, sims, 1, False, seed, max_memory_mb=1)
+        out["mcts_gc/%s" % gs] = dict(r, sizeof_search_node=ref_lib.sizeof_search_node())
+    return out
+
+
+@pytest.mark.parametrize("gs,prefix,sims,nroll,solve,seed", CASES, ids=["%s-%d" % (c[0], c[2]) for c in CASES])
+def test_oracle_mcts_equals_reference_mctsbot_bitwise(gs, prefix, sims, nroll, solve, seed):
+    ref = expected("mcts/%s-%d" % (gs, sims))
+    mine = oracle_mcts(start(OracleGame(gs), gs, prefix, seed), 2.0, sims, nroll, solve, seed, reference_rng=True)
     assert [c[0] for c in mine["children"]] == [c[0] for c in ref["children"]]          # same shuffled child order
     assert [c[1] for c in mine["children"]] == [c[1] for c in ref["children"]]          # visit counts
     assert [c[2] for c in mine["children"]] == [c[2] for c in ref["children"]]          # total rewards, exact doubles
@@ -56,18 +73,17 @@ def test_oracle_mcts_equals_reference_mctsbot_bitwise(gs, prefix, sims, nroll, s
     assert mine["root_visits"] == ref["root_visits"]
 
 
-@pytest.mark.parametrize("gs,sims,seed", [("connect_four", 12000, 3), ("hex(board_size=4)", 9000, 5)])
+@pytest.mark.parametrize("gs,sims,seed", GC_CASES)
 def test_oracle_garbage_collection_equals_reference_bitwise(gs, sims, seed):
     """MCTSBot's node budget (max_memory_mb -> max_nodes_, mcts.cc:205-231) and GarbageCollect (mcts.cc:441-482): with
     max_memory_mb = 1 the tree is collected several times inside these searches; the oracle must prune the same nodes at
     the same simulations (same gc_limit_ trajectory), i.e. reproduce the final root statistics bit for bit."""
-    rg, og = ref_lib.RefGame(gs), OracleGame(gs)
-    rs, os_ = rg.new_initial_state(), og.new_initial_state()
-    max_nodes = (1 << 20) // ref_lib.sizeof_search_node() + 1
-    ref = ref_lib.ref_mcts(rg, rs, 2.0, sims, 1, False, seed, max_memory_mb=1)
+    ref = expected("mcts_gc/%s" % gs)
+    os_ = OracleGame(gs).new_initial_state()
+    max_nodes = (1 << 20) // ref["sizeof_search_node"] + 1
     mine = oracle_mcts(os_, 2.0, sims, 1, False, seed, reference_rng=True, max_nodes=max_nodes)
     assert mine["gc_runs"] >= 2, mine["gc_runs"]
-    assert mine["children"] and [c[:3] for c in mine["children"]] == [tuple(c) for c in ref["children"]]
+    assert mine["children"] and [list(c[:3]) for c in mine["children"]] == ref["children"]
     assert mine["best_action"] == ref["best_action"] and mine["root_visits"] == ref["root_visits"]
     # and the budget changes the search: without it the statistics differ
     free = oracle_mcts(os_, 2.0, sims, 1, False, seed, reference_rng=True)

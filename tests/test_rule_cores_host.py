@@ -132,14 +132,71 @@ def test_rule_core_lockstep_vs_oracle(gs, n):
     _lockstep(gs, n, OracleGame)
 
 
-@pytest.mark.parametrize("gs,n", [(g, max(8, k // 3)) for g, k in GAMES], ids=[g for g, _ in GAMES])
+REF_GAMES = [(g, max(8, k // 3)) for g, k in GAMES]
+
+
+@pytest.mark.parametrize("gs,n", REF_GAMES, ids=[g for g, _ in GAMES])
 def test_rule_core_lockstep_vs_unmodified_reference(gs, n):
-    """The same lock-step play with the UNMODIFIED reference (oracle/_ref) as the checker: the code the CUDA kernels are
-    built from against open_spiel's own State classes, in the CPU suite."""
+    """The same lock-step play with the UNMODIFIED reference as the checker: the code the CUDA kernels are built from
+    against open_spiel's own State classes, in the CPU suite.  The reference's side is stored (tests/reference_golden.py):
+    a digest of everything _lockstep compares, along the same games."""
+    from reference_golden import Digest, expected
+    want = expected("rule_cores/" + gs)
+    emu = Emu(gs, n)
+    info = emu.info
+    P, has_info = info.num_players, want["has_info"]
+    rng = np.random.RandomState(sum(map(ord, gs)) % 997)
+    d = Digest([info.num_distinct_actions, info.max_game_length, info.num_players, info.observation_tensor_size])
+    for ply in range(info.max_game_length + 8):
+        cur, term, rets = emu.status()
+        legal = emu.legal()
+        obs = [emu.tensor(p, 0) for p in range(P)]
+        ist = [emu.tensor(p, 1) for p in range(P)] if has_info else None
+        actions = np.full(n, -1, dtype=np.int32)
+        for i in range(n):
+            _record(d, cur[i], term[i], legal[i], rets[i].tolist(), [o[i] for o in obs], ist and [t[i] for t in ist])
+            if not term[i]:
+                actions[i] = legal[i][rng.randint(len(legal[i]))]
+        if (actions < 0).all():
+            break
+        emu.apply(actions)
+        assert emu.errors() == 0
+    else:
+        raise AssertionError("games did not end")
+    assert d.hexdigest() == want["digest"]
+
+
+def _record(d, cur, term, legal, rets, obs, ist):
+    d.add(int(cur), bool(term), legal, [float(x).hex() for x in rets], obs, ist)
+
+
+def reference_golden():
+    """The reference's side of test_rule_core_lockstep_vs_unmodified_reference: its states played the same way."""
     import ref_lib
-    if not ref_lib.available():
-        pytest.skip("oracle/_ref not built")
-    _lockstep(gs, n, ref_lib.RefGame)
+    from reference_golden import Digest
+    out = {}
+    for gs, n in REF_GAMES:
+        g = ref_lib.RefGame(gs)
+        rng = np.random.RandomState(sum(map(ord, gs)) % 997)
+        has_info = g.information_state_tensor_size > 0
+        P = g.num_players
+        d = Digest([g.num_distinct_actions, g.max_game_length, g.num_players, g.observation_tensor_size])
+        states = [g.new_initial_state() for _ in range(n)]
+        while True:
+            actions = []
+            for st in states:
+                _record(d, st.current_player(), st.is_terminal(), st.legal_actions(), st.returns(),
+                        [st.observation_tensor(p) for p in range(P)],
+                        [st.information_state_tensor(p) for p in range(P)] if has_info else None)
+                la = st.legal_actions()
+                actions.append(None if st.is_terminal() else la[rng.randint(len(la))])
+            if all(a is None for a in actions):
+                break
+            for st, a in zip(states, actions):
+                if a is not None:
+                    st.apply_action(a)
+        out["rule_cores/" + gs] = {"digest": d.hexdigest(), "has_info": has_info}
+    return out
 
 
 def _lockstep(gs, n, checker):

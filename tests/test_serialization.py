@@ -1,6 +1,8 @@
-"""CPU: the text formats of open_spiel_b200/serialization.py against the UNMODIFIED reference (oracle/_ref):
-information-state strings rebuilt from tensors, hex-float doubles, CFRSolverBase::Serialize / DeserializeCFRSolver in both
-directions (the reference loads what we write; we parse what it writes), State::Serialize."""
+"""CPU: the text formats of open_spiel_b200/serialization.py against the UNMODIFIED reference: information-state strings
+rebuilt from tensors, hex-float doubles, CFRSolverBase::Serialize / DeserializeCFRSolver in both directions (the reference
+loads what we write; we parse what it writes), State::Serialize.  The reference's side is stored (tests/reference_golden.py);
+the CFR tables behind it come from the oracle's CFRSolver, which reproduces the reference's bit for bit
+(test_cfr_oracle.py)."""
 import ctypes
 import random
 import struct
@@ -9,10 +11,8 @@ import numpy as np
 import pytest
 
 from open_spiel_b200 import serialization as ser
-from oracle_lib import OracleGame, infostate_tensors
-import ref_lib
-
-needs_ref = pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not built")
+from oracle_lib import OracleCFR, OracleGame, infostate_tensors
+from reference_golden import digest, expected
 
 
 def test_hex_double_is_printf_percent_a():
@@ -61,52 +61,88 @@ def _layout_from(ref_table, name):
     return keys, t
 
 
-@needs_ref
-@pytest.mark.parametrize("name,iters", [("kuhn_poker", 37), ("leduc_poker", 6)])
-def test_cfr_solver_text_format_both_directions(name, iters):
-    rg = ref_lib.RefGame(name)
-    ref = ref_lib.RefCFR(rg)
-    ref.iterate(iters)
-    text = ref_lib.cfr_serialize(ref)
-    # (1) we parse what the reference writes
-    parsed = ser.deserialize_cfr_solver(text)
-    assert parsed["game"] == ref_lib.game_to_string(rg) and parsed["solver_type"] == "CFRSolver" and parsed["iteration"] == iters
-    assert parsed["table"] == ref.table()
-    # (2) we write what the reference writes: same header, same set of table entries byte for byte (the reference emits
-    # its unordered_map in hash order, so only the order of entries may differ)
-    keys, layout = _layout_from(ref.table(), name)
-    assert ser.table_keys(name, layout) == keys
-    mine = ser.serialize_cfr_solver(ref_lib.game_to_string(rg), "CFRSolver", iters, keys, layout)
-    head_r, _, vals_r = text.partition("[SolverValuesTable]\n")
-    head_m, _, vals_m = mine.partition("[SolverValuesTable]\n")
-    assert head_m == head_r
-    pairs = lambda v: sorted(zip(v.split(ser.DELIMITER)[0::2], v.split(ser.DELIMITER)[1::2]))   # noqa: E731
-    assert pairs(vals_m) == pairs(vals_r)
-    # (3) the reference loads what we write, and continues training from it exactly like the original
-    loaded = ref_lib.cfr_deserialize(rg, mine)
-    assert loaded.table() == ref.table()
-    loaded.iterate(3)
-    ref.iterate(3)
-    assert loaded.table() == ref.table()
-    # (4) and back into flat arrays in a given row order (CFRSolver.load_table's arguments)
-    r, c, p = ser.table_arrays_from(parsed["table"], keys, layout)
-    assert np.array_equal(r, layout["regrets"]) and np.array_equal(c, layout["cum_policy"]) and np.array_equal(p, layout["cur_policy"])
+CFR_CASES = [("kuhn_poker", 37), ("leduc_poker", 6)]
+STATE_GAMES = ["connect_four", "go(board_size=5)", "kuhn_poker", "leduc_poker", "breakthrough"]
 
 
-@needs_ref
-@pytest.mark.parametrize("gs", ["connect_four", "go(board_size=5)", "kuhn_poker", "leduc_poker", "breakthrough"])
-def test_state_serialize_format(gs):
-    rng = random.Random(3)
-    rg = ref_lib.RefGame(gs)
-    st = rg.new_initial_state()
+def entries_digest(text):
+    """The header of a serialized solver and the set of its table entries (the reference emits its unordered_map in hash
+    order, so only the order of entries may differ)."""
+    head, _, vals = text.partition("[SolverValuesTable]\n")
+    parts = vals.split(ser.DELIMITER)
+    return digest(head, sorted(zip(parts[0::2], parts[1::2])))
+
+
+def table_digest(t):
+    return digest({k: [v["legal"], v["regrets"], v["cum_policy"], v["cur_policy"]] for k, v in t.items()})
+
+
+def random_history(game, rng, plies=12):
+    st = game.new_initial_state()
     hist = []
-    for _ in range(12):
+    for _ in range(plies):
         if st.is_terminal():
             break
         a = rng.choice(st.legal_actions())
         st.apply_action(a)
         hist.append(a)
+    return st, hist
+
+
+def reference_golden():
+    import ref_lib
+    out = {}
+    for name, iters in CFR_CASES:
+        rg = ref_lib.RefGame(name)
+        ref = ref_lib.RefCFR(rg)
+        ref.iterate(iters)
+        text = ref_lib.cfr_serialize(ref)
+        keys, layout = _layout_from(ref.table(), name)
+        mine = ser.serialize_cfr_solver(ref_lib.game_to_string(rg), "CFRSolver", iters, keys, layout)
+        loaded = ref_lib.cfr_deserialize(rg, mine)           # the reference loads what we write ...
+        first = table_digest(loaded.table())
+        loaded.iterate(3)                                     # ... and continues training from it
+        out["serialization/cfr/" + name] = {"game": ref_lib.game_to_string(rg), "text": entries_digest(text),
+                                            "parsed": table_digest(ser.deserialize_cfr_solver(text)["table"]),
+                                            "loaded": first, "loaded_plus_3": table_digest(loaded.table())}
+    for gs in STATE_GAMES:
+        rg = ref_lib.RefGame(gs)
+        st, hist = random_history(rg, random.Random(3))
+        text = ref_lib.state_serialize(st)
+        back = ref_lib.deserialize_state(rg, text)
+        out["serialization/state/" + gs] = {"text": text, "history": back.history(), "to_string": back.to_string()}
+    return out
+
+
+@pytest.mark.parametrize("name,iters", CFR_CASES)
+def test_cfr_solver_text_format_both_directions(name, iters):
+    want = expected("serialization/cfr/" + name)
+    o = OracleCFR(OracleGame(name))              # the reference's CFRSolver tables, bit for bit (test_cfr_oracle.py)
+    o.iterate(iters)
+    table = o.table()
+    # (1) we write what the reference writes: same header, same set of table entries byte for byte
+    keys, layout = _layout_from(table, name)
+    assert ser.table_keys(name, layout) == keys
+    mine = ser.serialize_cfr_solver(want["game"], "CFRSolver", iters, keys, layout)
+    assert entries_digest(mine) == want["text"]
+    # (2) so we parse what the reference writes: its text is ours up to the order of entries
+    parsed = ser.deserialize_cfr_solver(mine)
+    assert parsed["game"] == want["game"] and parsed["solver_type"] == "CFRSolver" and parsed["iteration"] == iters
+    assert table_digest(parsed["table"]) == want["parsed"] == table_digest(table)
+    # (3) the reference loads what we write, and continues training from it exactly like the original
+    assert want["loaded"] == table_digest(table)
+    o.iterate(3)
+    assert want["loaded_plus_3"] == table_digest(o.table())
+    # (4) and back into flat arrays in a given row order (CFRSolver.load_table's arguments)
+    r, c, p = ser.table_arrays_from(parsed["table"], keys, layout)
+    assert np.array_equal(r, layout["regrets"]) and np.array_equal(c, layout["cum_policy"]) and np.array_equal(p, layout["cur_policy"])
+
+
+@pytest.mark.parametrize("gs", STATE_GAMES)
+def test_state_serialize_format(gs):
+    want = expected("serialization/state/" + gs)
+    st, hist = random_history(OracleGame(gs), random.Random(3))
     text = ser.serialize_state(hist)
-    assert text == ref_lib.state_serialize(st)
-    back = ref_lib.deserialize_state(rg, text)
-    assert back.history() == hist and back.to_string() == st.to_string()
+    assert text == want["text"]
+    # the reference's state deserialized from that text
+    assert want["history"] == hist and want["to_string"] == st.to_string()

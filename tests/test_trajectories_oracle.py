@@ -3,14 +3,16 @@ RecordBatchedTrajectory (algorithms/trajectories.cc:98-200, built by oracle/ref_
 random streams, so every reference episode is lined up by replaying its own action sequence through the oracle
 recorder (forced mode): the chance outcomes, which the reference does not record, are read off the information-state
 tensors (private card one-hots of both players, public card one-hot in leduc's second round).  All recorded fields
-and the padding convention must then agree exactly."""
+and the padding convention must then agree exactly.  The reference's batch is stored (tests/reference_golden.py): the action
+sequences read off each episode, and a digest of every recorded field."""
 import numpy as np
 import pytest
 
 from oracle_lib import OracleGame, oracle_record_trajectory
-import ref_lib
+from reference_golden import Digest, expected
 
-pytestmark = pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not built")
+FIELDS = ("legal_actions", "observations", "actions", "player_ids", "valid", "next_is_terminal", "rewards", "player_policies")
+B = 300
 
 
 def _kuhn_sequence(ep):
@@ -42,24 +44,40 @@ def _leduc_sequence(ep):
     return seq
 
 
-@pytest.mark.parametrize("name,T,sequence", [("kuhn_poker", 5, _kuhn_sequence), ("leduc_poker", 10, _leduc_sequence)])
+CASES = [("kuhn_poker", 5, _kuhn_sequence), ("leduc_poker", 10, _leduc_sequence)]
+
+
+def reference_golden():
+    import ref_lib
+    out = {}
+    for name, T, sequence in CASES:
+        ref = ref_lib.ref_record_batched_trajectory(ref_lib.RefGame(name), B, seed=1234, T=T)
+        d = Digest()
+        seqs = []
+        for b in range(B):
+            ep = {k: v[b] for k, v in ref.items()}
+            seqs.append([int(x) for x in sequence(ep)])
+            d.add([ep[k] for k in FIELDS])
+        out["trajectories/" + name] = {"sequences": seqs, "digest": d.hexdigest()}
+    return out
+
+
+@pytest.mark.parametrize("name,T,sequence", CASES)
 def test_oracle_recorder_reproduces_reference_episodes(name, T, sequence):
-    B = 300
-    rg, og = ref_lib.RefGame(name), OracleGame(name)
-    ref = ref_lib.ref_record_batched_trajectory(rg, B, seed=1234, T=T)
+    want = expected("trajectories/" + name)
+    og = OracleGame(name)
+    d = Digest()
     lengths = set()
-    for b in range(B):
-        ep = {k: v[b] for k, v in ref.items()}
-        forced = sequence(ep)
+    for forced in want["sequences"]:
         mine = oracle_record_trajectory(og.new_initial_state(), seed=0, lane=0, T=T, forced=forced)
-        assert mine["length"] == int(ep["valid"].sum())
+        assert mine["length"] == int(mine["valid"].sum())
+        assert sequence(mine) == forced          # the episode's tensors name the same chance outcomes and actions
         lengths.add(mine["length"])
-        for k in ("legal_actions", "observations", "actions", "player_ids", "valid", "next_is_terminal", "rewards"):
-            assert np.array_equal(mine[k], ep[k]), (name, b, k)
         # player_policies of the uniform policy: 1/#legal on the legal actions; padding rows all ones (ResizeFields)
-        la = ep["legal_actions"].astype(np.float64)
-        expect = np.where(ep["valid"][:, None] == 1, la / la.sum(-1, keepdims=True), 1.0)
-        assert np.array_equal(ep["player_policies"], expect)
+        la = mine["legal_actions"].astype(np.float64)
+        mine["player_policies"] = np.where(mine["valid"][:, None] == 1, la / la.sum(-1, keepdims=True), 1.0)
+        d.add([np.asarray(mine[k]) for k in FIELDS])
+    assert len(want["sequences"]) == B and d.hexdigest() == want["digest"]
     assert len(lengths) > 1          # ragged batch: the padding convention was exercised
 
 
