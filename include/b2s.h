@@ -114,7 +114,7 @@ int b2s_legal_list(void* batch, int16_t* actions_d, int32_t* counts_d, int32_t s
 
 /* State::CurrentPlayer / IsTerminal / Returns (spiel.h:330,447,470).  Any output may be NULL.
  * current_player: >=0 player, -1 chance (kChancePlayerId), -4 terminal (kTerminalPlayerId).
- * returns_d is [n][num_players] float32. */
+ * returns_d is [n][num_players] float32; like every float output it needs 4-byte alignment only. */
 int b2s_status(void* batch, int8_t* current_player_d, uint8_t* terminal_d, float* returns_d, int64_t n, void* stream);
 
 /* State::ObservationTensor(player) (spiel.cc:908-925): [n][observation_tensor_size] float32,

@@ -149,6 +149,20 @@ __global__ void __launch_bounds__(kBlock) k_legal_list(Ctx ctx, typename R::Cfg 
   counts[i] = k;
 }
 
+// Returns row i of a [n][num_players] float buffer.  Two players: one 8-byte store per lane when the buffer allows it; the
+// C ABI promises only float (4-byte) alignment, so a buffer at an odd float offset takes two 4-byte stores (the test is on
+// the base pointer, hence uniform over the launch).
+template <class R>
+__device__ __forceinline__ void store_returns(float* __restrict__ rets, long long i, const float* r, const typename R::Cfg& cfg) {
+  if (R::kPlayers == 2) {
+    if (((unsigned long long)rets & 7ull) == 0) reinterpret_cast<float2*>(rets)[i] = make_float2(r[0], r[1]);
+    else { rets[2 * i] = r[0]; rets[2 * i + 1] = r[1]; }
+  } else {
+    const int np = rule_num_players<R>(cfg);
+    for (int p = 0; p < np; ++p) rets[i * np + p] = r[p];
+  }
+}
+
 template <class R, int ILP>
 __global__ void __launch_bounds__(kBlock) k_status(Ctx ctx, typename R::Cfg cfg, signed char* __restrict__ cur, unsigned char* __restrict__ term, float* __restrict__ rets, long long n) {
   long long base = (long long)blockIdx.x * (kBlock * ILP) + threadIdx.x;
@@ -168,8 +182,7 @@ __global__ void __launch_bounds__(kBlock) k_status(Ctx ctx, typename R::Cfg cfg,
     if (rets) {
       float r[R::kPlayers];
       R::returns(s[j], cfg, r);
-      if (R::kPlayers == 2) reinterpret_cast<float2*>(rets)[i] = make_float2(r[0], r[1]);
-      else { const int np = rule_num_players<R>(cfg); for (int p = 0; p < np; ++p) rets[i * np + p] = r[p]; }
+      store_returns<R>(rets, i, r, cfg);
     }
   }
 }
@@ -204,8 +217,7 @@ __global__ void __launch_bounds__(kBlock) k_step_fused(Ctx ctx, typename R::Cfg 
       if (rets) {
         float r[R::kPlayers];
         R::returns(s[j], cfg, r);
-        if (R::kPlayers == 2) reinterpret_cast<float2*>(rets)[i] = make_float2(r[0], r[1]);
-        else { const int np = rule_num_players<R>(cfg); for (int p = 0; p < np; ++p) rets[i * np + p] = r[p]; }
+        store_returns<R>(rets, i, r, cfg);
       }
       if (mask) {
         if (t) { for (int w = 0; w < R::kMaskWords; ++w) m[w] = 0; }

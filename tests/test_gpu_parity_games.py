@@ -59,11 +59,22 @@ GAMES = [
     ("leduc_poker(players=4)", 256),
     ("leduc_poker(starting_player=1)", 256),
 ]
+# the same games again at several blocks of the ILP kernels with a ragged last warp: 2085 = 2 * (256 * 4) + 37 lanes at
+# ILP 4, 1061 = 2 * (256 * 2) + 37 at ILP 2
+MULTI_BLOCK = [
+    ("tic_tac_toe", 2085),
+    ("connect_four", 2085),
+    ("kuhn_poker", 2085),
+    ("leduc_poker", 2085),
+    ("breakthrough", 1061),
+    ("othello", 1061),
+]
 INFO_STATE = {"kuhn_poker", "kuhn_poker(players=3)", "kuhn_poker(players=5)", "leduc_poker", "leduc_poker(starting_player=1)",
               "leduc_poker(players=3)", "leduc_poker(players=4)"}
 
 
-@pytest.mark.parametrize("game_string,lanes", GAMES, ids=[g for g, _ in GAMES])
+@pytest.mark.parametrize("game_string,lanes", GAMES + MULTI_BLOCK,
+                         ids=[g for g, _ in GAMES] + ["%s-%d" % (g, n) for g, n in MULTI_BLOCK])
 def test_lockstep_random_games(game_string, lanes):
     steps = lockstep(game_string, n_lanes=lanes, seed=1234, check_info_state=game_string in INFO_STATE)
     assert steps >= lanes
